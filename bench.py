@@ -15,6 +15,8 @@ roofline: all kernels of one op forward / backward (our .so), algorithmic bytes 
           CUDA-event time of those launches (L2 flushed between iterations).
 --impl reference : the reference module's CPU path (oracle module port; the Python reference cannot
           travel to the GPU box) on the host cores, bounded sample of the same workload.
+--dump-outputs DIR : after the timed op steps, rank 0 writes what the last step's last recurrence returned (out, lse, dq,
+          dk, dv) as DIR/<name>.npy in float32, for comparing two builds on the same seeded inputs (see dump_outputs).
 """
 from __future__ import annotations
 
@@ -220,6 +222,24 @@ def workload_name():
             f"(1x1 convs + op + residual) on the same shape")
 
 
+DUMP_MAX_ELEMS = 1 << 21        # per array (8 MB as float32): the five op outputs stay under 64 MB in all
+
+
+def dump_outputs(path, tensors):
+    """Write each tensor as ``path/<name>.npy`` in float32.  A tensor of at most DUMP_MAX_ELEMS elements is written whole in
+    its logical (NCHW) shape; a larger one as the 1-D sample ``t.contiguous().view(-1)[idx]`` with
+    ``idx = sorted(numpy.random.default_rng(0).choice(t.numel(), DUMP_MAX_ELEMS, replace=False))``, so every run of the
+    same shape samples the same elements."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in tensors.items():
+        t = t.detach().float().contiguous()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_MAX_ELEMS, replace=False))
+            t = t.view(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
+
+
 def time_events(fn, steps, warmup, barrier=None, finish=None):
     """finish(): joins side streams into the current stream before the closing event (pipelined e2e)."""
     for _ in range(warmup):
@@ -367,16 +387,22 @@ def run_ours(args):
         q, k, v, do = (t.contiguous(memory_format=torch.channels_last) for t in (q, k, v, do))
     op_layout = "channels_last" if not q.is_contiguous() else "nchw"
 
+    last = {}                                       # what the latest step returned (for --dump-outputs)
+
     def step_op():                                  # R sequential op applications, forward + backward
         for _ in range(R):
             out, lse = cca_forward(q, k, v, impl=args.kernels)
-            cca_backward(do, q, k, v, out, lse, impl=args.kernels)
+            dq, dk, dv = cca_backward(do, q, k, v, out, lse, impl=args.kernels)
+        last.update(out=out, lse=lse, dq=dq, dk=dk, dv=dv)
 
     # ---- main timed region: op level, resident ------------------------------------------------------
     n0 = capi.launch_count()
     with ClockSampler(local_rank) as clk:
         ms = time_events(step_op, args.steps, args.warmup, barrier)
     launches = (capi.launch_count() - n0) * args.steps // (args.steps + args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    last.clear()
     ms = max_over_ranks(ms)
     px = B * H * W * world
     value = px / (ms * 1e-3)
@@ -519,7 +545,10 @@ def main():
     ap.add_argument("--kernels", default="auto", choices=["auto", "simt", "tc"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-train", action="store_true", help="skip the ResNet101+RCCA train-step leg (BASELINE configs[2], [3])")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed op step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(3, args.warmup)
     if args.impl == "reference":
         run_reference(args)

@@ -84,3 +84,24 @@ def test_qkv_projection_node_matches_the_three_convs():
         assert (o - r).abs().max().item() <= 1e-12
     for a, b in zip(got, want):
         assert a.shape == b.shape and (a - b).abs().max().item() <= 1e-10
+
+
+def test_dump_outputs_writes_whole_or_fixed_samples_within_64mb(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 .npy files, small arrays whole in their NCHW shape, large ones as the documented
+    seeded sample (same indices on every run), and the five op outputs of the flagship shape under 64 MB in all."""
+    import numpy as np
+    import bench
+    B, C, H, W = (bench.CFG[n] for n in "BCHW")
+    numels = [B * C * H * W, B * H * W, B * C // 8 * H * W, B * C // 8 * H * W, B * C * H * W]    # out, lse, dq, dk, dv
+    assert sum(4 * min(n, bench.DUMP_MAX_ELEMS) for n in numels) <= 64 << 20
+    monkeypatch.setattr(bench, "DUMP_MAX_ELEMS", 100)
+    big = torch.randn(2, 8, 5, 6).contiguous(memory_format=torch.channels_last)
+    small = torch.randn(2, 5, 6, dtype=torch.float64)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"big": big, "small": small})
+    got = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in ("big", "small")}
+    assert all(v.dtype == np.float32 for v in got.values())
+    assert got["small"].shape == (2, 5, 6) and np.array_equal(got["small"], small.float().numpy())
+    idx = np.sort(np.random.default_rng(0).choice(big.numel(), 100, replace=False))
+    assert np.array_equal(got["big"], big.contiguous().view(-1).numpy()[idx])
+    assert all(np.array_equal(got[n], np.load(tmp_path / "b" / f"{n}.npy")) for n in got)

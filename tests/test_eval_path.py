@@ -118,9 +118,9 @@ def test_load_model_semantics(tmp_path):
     m, missing, unexpected = ev.load_model(_Tiny(), str(f))
     assert not missing and not unexpected and torch.equal(m.a.weight, src.a.weight)
     # 3. is_restore: keys get the 'module.' prefix of a DataParallel wrapper (pyt_utils.py:58-63)
-    wrapped = nn.DataParallel(_Tiny())
+    wrapped = nn.DataParallel(_Tiny())               # with one visible GPU this moves the module to cuda:0
     m, missing, unexpected = ev.load_model(wrapped, sd, is_restore=True)
-    assert not missing and not unexpected and torch.equal(m.module.a.weight, src.a.weight)
+    assert not missing and not unexpected and torch.equal(m.module.a.weight.cpu(), src.a.weight)
     # 4. non-strict: missing and unexpected keys are reported, the rest is loaded (pyt_utils.py:65-77)
     part = OrderedDict((k, v) for k, v in sd.items() if not k.startswith("b."))
     part["head.extra"] = torch.zeros(1)
